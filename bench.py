@@ -2,7 +2,7 @@
 """bench.py — encode->decode throughput of the colour-modem hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload pald576|ntsc3d600|sweep1080] [--frames F]
+                    [--workload pald576|ntsc3d600|sweep1080] [--frames F] [--dump-outputs DIR]
 
 Workloads
   pald576    (default; BASELINE configs[1], the configuration the metric is quoted on): standard 625-line PAL, PAL-D
@@ -33,6 +33,7 @@ import argparse
 import json
 import os
 import queue
+import re
 import subprocess
 import sys
 import threading
@@ -64,7 +65,13 @@ def parse():
     ap.add_argument('--e2e-seconds', type=float, default=1.5, help='target length of each end-to-end timed region')
     ap.add_argument('--no-extras', action='store_true', help='skip the short runs of the other BASELINE configs')
     ap.add_argument('--no-cpu', action='store_true', help='skip the CPU baseline beside the GPU number')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (rank 0) as DIR/<name>.npy in float32, a fixed seeded '
+                         'sample of its rows of at most 64 MB, so that two builds can be compared output for output')
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours (the reference arm keeps no frames)')
+    return a
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -327,6 +334,27 @@ def timed_steps(D, step, steps, warmup):
     return D.max(e0.elapsed_time(e1)), t_begin, t_end
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(dirname, first_frame, budget=DUMP_BYTES, prefix='', **arrays):
+    """DIR/<prefix><name>.npy (float32) for each device array [frames, rows, ...] of one step, all at the same rows: a
+    seeded choice of its rows (the same for the same arguments) that fits `budget` bytes; DIR/<prefix>frame_index.npy and
+    DIR/<prefix>row_index.npy (float64) say which, in absolute frame numbers."""
+    import numpy as np
+    import torch
+    n, h = next(iter(arrays.values())).shape[:2]
+    per_row = 16 + sum(4 * a[0, 0].numel() for a in arrays.values())
+    k = min(n * h, (budget - 4096) // per_row)
+    pick = np.sort(np.random.default_rng(0).choice(n * h, k, replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, prefix + 'frame_index.npy'), (first_frame + pick // h).astype(np.float64))
+    np.save(os.path.join(dirname, prefix + 'row_index.npy'), (pick % h).astype(np.float64))
+    for name, a in arrays.items():
+        sample = a.reshape(n * h, *a.shape[2:])[torch.from_numpy(pick).to(a.device)].cpu().numpy()
+        np.save(os.path.join(dirname, prefix + name + '.npy'), sample.astype(np.float32))
+
+
 def tiled_frames(torch, dev, n, hh, ww, first_frame, seed=0, distinct=16):
     """[n, hh, ww, 3] u8 on the device: `distinct` synthetic frames tiled (content does not affect the data-independent
     kernels); returns (device tensor, numpy base)."""
@@ -446,6 +474,8 @@ def run_pald(args, D, cpu_line):
     ms, t_begin, t_end = timed_steps(D, step, args.steps, warmup)
     launches = (N.launch_count() - launches0) * args.steps // (args.steps + warmup)
     clocks = sampler.stop(t_begin, t_end) if D.rank == 0 else None
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, first_frame, composite=comp, rgb=out)
 
     # ---- per-kernel device time (CUDA events around every launch), as run -----------------------------------------------
     modem.timing(True)
@@ -688,6 +718,8 @@ def run_ntsc3d600(args, D, cpu_line):
     ms, t_begin, t_end = timed_steps(D, step, args.steps, warmup)
     launches = (N.launch_count() - launches0) * args.steps // (args.steps + warmup)
     clocks = sampler.stop(t_begin, t_end) if D.rank == 0 else None
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, lo, composite=comp, rgb=out)
     if D.rank == 0:
         j = min(3, hi - lo - 1)
         lsb_c, lsb_o = parity_check('ntsc_3d', 'NTSC', hh, ww, lo + j, rgb[j].cpu().numpy(), comp[j].cpu().numpy(),
@@ -759,6 +791,14 @@ def run_sweep1080(args, D, cpu_line):
     ms, t_begin, t_end = timed_steps(D, step, args.steps, warmup)
     launches = (N.launch_count() - launches0) * args.steps // (args.steps + warmup)
     clocks = sampler.stop(t_begin, t_end) if D.rank == 0 else None
+    if args.dump_outputs and D.rank == 0:
+        # presets share output buffers, so each one's pass of the timed step is replayed and written before the next
+        for name, m in modems:
+            c, o = bufs[(m.composite_width, m.output_width)]
+            m.encode_frames(rgb, first_frame=lo, out=c)
+            m.decode_frames(c, first_frame=lo, out=o)
+            dump_outputs(args.dump_outputs, lo, DUMP_BYTES // len(modems), re.sub(r'[^A-Za-z0-9]+', '_', name) + '.',
+                         composite=c, rgb=o)
     step(record=True)
     D.barrier()
     rows = []

@@ -12,12 +12,13 @@ Rules (see DESIGN.md):
 
 Parity pin: the reference ships no tests or golden vectors, so the oracle is
 pinned against *outputs of the reference itself*: ``tests/golden/make_golden.py``
-imports ``/root/reference`` (with the scipy ``iirdesign`` validation shim
-described in SURVEY.md §8c), runs ``ImageModem.modulate/demodulate`` for every
-supported composition/preset and commits the u8 frames plus a few float64
-lines under ``tests/golden/``.  ``tests/test_oracle_golden.py`` checks this
-oracle against those fixtures (CPU-only), and ``tests/test_oracle_vs_reference.py``
-re-checks live whenever ``/root/reference`` is importable.
+imports a checkout of the reference named by ``COLOR_MODEM_REFERENCE`` (with the
+scipy ``iirdesign`` validation shim described in SURVEY.md §8c), runs
+``ImageModem.modulate/demodulate`` for every supported composition/preset and
+commits the u8 frames plus a few float64 lines under ``tests/golden/``.
+``tests/test_oracle_golden.py`` checks this oracle against those fixtures
+(CPU-only), and ``tests/test_oracle_vs_reference.py`` re-checks live whenever
+``COLOR_MODEM_REFERENCE`` is set.
 
 Third-party arithmetic: the reference calls ``scipy.signal`` (``lfilter``,
 ``resample_poly``, ``iirdesign``, ``iirfilter``, ``group_delay``, ``freqz``;

@@ -5,6 +5,10 @@ Frames are small (24 rows) with an explicit line standard so the fixtures stay a
 ``LineConfig((W, 24), standard)`` is a legal reference configuration (line.py:50-55).
 """
 import collections
+import hashlib
+import os
+
+import numpy as np
 
 Case = collections.namedtuple('Case', 'kind variant width height standard chroma_avg frame seed content notch opt')
 # notch: Q of the luma notch of the comb decoders (comb.py:18-20), 0 = off
@@ -118,8 +122,69 @@ GOLDEN_CASES = [
 
 FLOAT_ROWS = (1, 10, 22)   # rows whose float64 composite / RGB lines are stored: field top, interior, field bottom
 
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+# The decoded frame `rgb_u8` of a whole-frame fixture does not compress below 1 MB, so it is stored in chunks of this many
+# rows: the first chunk in <id>.npz with the other arrays, chunk k in <id>.part<k>.npz.
+RGB_ROWS_PER_FILE = 192
+
 
 def case_id(c):
     return '%s-%s-%dx%d-%s%s-f%d-%s%s' % (c.kind, c.variant, c.width, c.height, c.standard,
                                           '-avg' if c.chroma_avg else '', c.frame, c.content,
                                           ('-notch%g' % c.notch if c.notch else '') + ('-' + c.opt if c.opt else ''))
+
+
+def save_golden(c, **arrays):
+    base = os.path.join(GOLDEN_DIR, case_id(c))
+    rgb = arrays.pop('rgb_u8')
+    np.savez_compressed(base + '.npz', rgb_u8=rgb[:RGB_ROWS_PER_FILE], **arrays)
+    for k, y in enumerate(range(RGB_ROWS_PER_FILE, rgb.shape[0], RGB_ROWS_PER_FILE), 1):
+        np.savez_compressed('%s.part%d.npz' % (base, k), rgb_u8=rgb[y:y + RGB_ROWS_PER_FILE])
+    return base + '.npz'
+
+
+def load_golden(c):
+    """The arrays of case c's fixture (comp_u8, rgb_u8, comp_f64, rgb_f64), the chunks of rgb_u8 joined."""
+    base = os.path.join(GOLDEN_DIR, case_id(c))
+    with np.load(base + '.npz') as f:
+        g = dict(f)
+    chunks, k = [g['rgb_u8']], 1
+    while os.path.exists('%s.part%d.npz' % (base, k)):
+        with np.load('%s.part%d.npz' % (base, k)) as f:
+            chunks.append(f['rgb_u8'])
+        k += 1
+    g['rgb_u8'] = np.concatenate(chunks)
+    return g
+
+
+# BASELINE configs 1-5 at their full size (tests/test_oracle_vs_reference.py).  A whole frame does not fit a fixture, so
+# full-<id>.npz holds the SHA-256 of each u8 frame (comp, rgb) with its shape, a few of its rows for diagnosis, and
+# `source`: 'reference' where the frames are the reference's own output, 'oracle' where they pin the oracle's output
+# until tests/golden/make_golden.py --full is run against the reference.
+FULL_CASES = [
+    Case('ntsc', 'NTSC', 720, 480, None, False, 0, 0, 'smooth'),          # BASELINE config 1
+    Case('pal_d', 'PAL', 720, 576, None, False, 0, 0, 'smooth'),          # BASELINE config 2
+    Case('ntsc_3d', 'NTSC', 720, 480, None, False, 599, 3, 'smooth'),     # BASELINE config 3 (last frame)
+    Case('secam', 'SECAM', 720, 576, None, True, 7, 4, 'noise'),          # BASELINE config 4a
+    Case('niir_hue', 'PAL', 720, 576, None, False, 999, 5, 'smooth'),     # BASELINE config 4b
+    Case('mac', 'D2MAC_7MHZ', 1920, 1080, 'GERBER_625', False, 2, 6, 'smooth'),   # BASELINE config 5 sample
+]
+FULL_SAMPLE_ROWS = 8
+
+
+def frame_digest(a):
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
+
+
+def save_full(c, comp_u8, rgb_u8, source):
+    rows = np.linspace(0, comp_u8.shape[0] - 1, FULL_SAMPLE_ROWS).round().astype(np.int64)
+    path = os.path.join(GOLDEN_DIR, 'full-%s.npz' % case_id(c))
+    np.savez_compressed(path, source=np.array(source), rows=rows,
+                        comp_sha256=frame_digest(comp_u8), comp_shape=np.array(comp_u8.shape), comp_rows=comp_u8[rows],
+                        rgb_sha256=frame_digest(rgb_u8), rgb_shape=np.array(rgb_u8.shape), rgb_rows=rgb_u8[rows])
+    return path
+
+
+def load_full(c):
+    with np.load(os.path.join(GOLDEN_DIR, 'full-%s.npz' % case_id(c))) as f:
+        return dict(f)

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run with -m gpu on the B200 box)')
-    config.addinivalue_line('markers', 'reference: needs /root/reference importable (builder container only)')
+    config.addinivalue_line('markers', 'reference: needs a checkout of the reference named by COLOR_MODEM_REFERENCE')
 
 
 def have_cuda():

@@ -10,7 +10,7 @@ sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, HERE)
 import oracle                                              # noqa: E402
 from oracle import frame as oframe                         # noqa: E402
-from cases import GOLDEN_CASES, case_id                    # noqa: E402
+from cases import GOLDEN_CASES, case_id, load_golden       # noqa: E402
 from product import BUILT_KINDS, make_modem                # noqa: E402
 from color_modem_b200.synth import synth_frames_u8         # noqa: E402
 
@@ -20,7 +20,7 @@ sel = sys.argv[1] if len(sys.argv) > 1 else ''
 for c in GOLDEN_CASES:
     if c.kind not in BUILT_KINDS or sel not in case_id(c):
         continue
-    g = np.load(os.path.join(HERE, 'golden', case_id(c) + '.npz'))
+    g = load_golden(c)
     rgb = synth_frames_u8(1, c.height, c.width, first_frame=c.frame, seed=c.seed, kind=c.content)[0]
     om = oracle.build(oracle.ModemSpec(c.kind, c.variant, c.width, c.height, c.standard, c.chroma_avg, c.notch, c.opt))
     rgb01 = rgb / 255.0

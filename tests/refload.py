@@ -1,7 +1,8 @@
-"""Load the read-only reference (/root/reference) for golden generation and live cross-checks.
+"""Load the reference, kFYatek/color_modem, for golden generation and live cross-checks.
 
-Only usable in the builder container; on the GPU box ``reference_available()`` is False and the
-tests that need it are skipped.  Nothing here is used by the product.
+The reference is not part of this repository: set COLOR_MODEM_REFERENCE to the directory of a checkout (the one
+holding the ``color_modem`` package).  Without it ``reference_available()`` is False and the tests that need it are
+skipped.  Nothing here is used by the product.
 """
 import contextlib
 import os
@@ -9,11 +10,11 @@ import sys
 
 import numpy as np
 
-REFERENCE_ROOT = '/root/reference'
+REFERENCE_ROOT = os.environ.get('COLOR_MODEM_REFERENCE', '')
 
 
 def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, 'color_modem'))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, 'color_modem'))
 
 
 class _Ref(object):

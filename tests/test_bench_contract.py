@@ -45,6 +45,33 @@ def test_workload_names_and_defaults():
     assert bench.BYTES_PER_FRAME == 3317760 and bench.DECODE_BYTES_PER_FRAME == 1658880
 
 
+def test_dump_outputs_is_a_fixed_sample_within_64_mb(tmp_path):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    n, h, w = 64, 576, 720
+    g = torch.Generator().manual_seed(1)
+    comp = torch.randint(0, 256, (n, h, w), dtype=torch.uint8, generator=g)
+    out = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, generator=g)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), 100, composite=comp, rgb=out)
+    bench.dump_outputs(str(tmp_path / 'c'), 100, bench.DUMP_BYTES // 16, 'one_preset.', composite=comp, rgb=out)
+    names = sorted(os.listdir(tmp_path / 'a'))
+    assert names == ['composite.npy', 'frame_index.npy', 'rgb.npy', 'row_index.npy']
+    assert sum(os.path.getsize(tmp_path / 'a' / f) for f in names) <= 64 * 10 ** 6
+    assert sum(os.path.getsize(tmp_path / 'c' / f) for f in os.listdir(tmp_path / 'c')) <= 64 * 10 ** 6 // 16
+    assert sorted(os.listdir(tmp_path / 'c')) == ['one_preset.' + f for f in names]
+    frames, rows = (np.load(tmp_path / 'a' / f) for f in ('frame_index.npy', 'row_index.npy'))
+    assert frames.dtype == rows.dtype == np.float64 and len(frames) == (64 * 10 ** 6 - 4096) // (16 + 4 * 4 * w)
+    assert len(np.unique(frames)) == n and ((frames - 100) * h + rows == np.unique((frames - 100) * h + rows)).all()
+    f, r = frames.astype(np.int64) - 100, rows.astype(np.int64)
+    for name, x in (('composite', comp), ('rgb', out)):
+        got = np.load(tmp_path / 'a' / (name + '.npy'))
+        assert got.dtype == np.float32 and np.array_equal(got, x.numpy()[f, r])
+        assert np.array_equal(got, np.load(tmp_path / 'b' / (name + '.npy')))
+
+
 def test_committed_bench_lines_carry_the_contract():
     """The lines bench.py printed on the B200 boxes (profiles/r2_bench*.json) have every key of the measurement contract: the base
     keys, `clocks`, `parity` within 1 LSB, `e2e` with its byte counts and the two beside-forms, `gpu_launches` > 0,

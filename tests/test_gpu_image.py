@@ -2,19 +2,16 @@
 ``.demodulate(img, frame)`` with PIL images (image.py:27-84) — against the bytes the reference itself produced
 (tests/golden/*.npz), including the automatic mode conversion of image.py:28-29,60-61 and the integer-width form of
 ``MacModem`` (mac.py:18-21)."""
-import os
-
 import numpy as np
 import pytest
 
-from cases import GOLDEN_CASES, case_id
+from cases import GOLDEN_CASES, case_id, load_golden
 from product import make_modem
 from color_modem_b200.image import ImageModem
 from color_modem_b200.synth import synth_frames_u8
 
 pytestmark = pytest.mark.gpu
 
-GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 PICK = {('pal_d', 'PAL', 720, 24, ''), ('ntsc_3d', 'NTSC', 720, 24, ''), ('secam', 'SECAM', 720, 24, ''),
         ('mac', 'D2MAC_7MHZ', 720, 24, ''), ('pal_s', 'PAL', 720, 24, ''), ('ntsc', 'NTSC', 720, 480, ''),
         ('pal_d', 'PAL', 720, 576, '')}
@@ -34,7 +31,7 @@ def _lsb(a, b):
 @pytest.mark.parametrize('c', CASES, ids=case_id)
 def test_pil_images_against_reference_bytes(c, cuda_required):
     from PIL import Image
-    g = np.load(os.path.join(GOLDEN_DIR, case_id(c) + '.npz'))
+    g = load_golden(c)
     rgb = synth_frames_u8(1, c.height, c.width, first_frame=c.frame, seed=c.seed, kind=c.content)[0]
     driver = ImageModem(make_modem(c))
     comp_img = driver.modulate(Image.fromarray(rgb, 'RGB'), c.frame)
@@ -49,7 +46,7 @@ def test_mode_conversion_like_the_reference(cuda_required):
     """image.py:28-29 / 60-61: any other PIL mode is converted to 'RGB' / 'L' first."""
     from PIL import Image
     c = [x for x in CASES if x.kind == 'pal_d' and x.height == 24][0]
-    g = np.load(os.path.join(GOLDEN_DIR, case_id(c) + '.npz'))
+    g = load_golden(c)
     rgb = synth_frames_u8(1, c.height, c.width, first_frame=c.frame, seed=c.seed, kind=c.content)[0]
     driver = ImageModem(make_modem(c))
     img = Image.fromarray(rgb, 'RGB')

@@ -3,21 +3,18 @@
   (b) the float64 oracle on the same seeded inputs.
 Tolerances are north_star's: fp32 kernels <= 1e-4 max abs error on the normalised composite and decoded planes
 and +-1 LSB on 8-bit output; the fp64 verification build <= 1e-9."""
-import os
-
 import numpy as np
 import pytest
 
 import conditioning
 import oracle
 from oracle import frame as oframe
-from cases import GOLDEN_CASES, case_id
+from cases import GOLDEN_CASES, case_id, load_golden
 from product import BUILT_KINDS, make_modem
 from color_modem_b200.synth import synth_frames_u8
 
 pytestmark = pytest.mark.gpu
 
-GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 CASES = [c for c in GOLDEN_CASES if c.kind in BUILT_KINDS]
 
 FP32_TOL = 1e-4
@@ -25,7 +22,7 @@ FP64_TOL = 1e-9
 
 
 def _inputs(c):
-    g = np.load(os.path.join(GOLDEN_DIR, case_id(c) + '.npz'))
+    g = load_golden(c)
     rgb = synth_frames_u8(1, c.height, c.width, first_frame=c.frame, seed=c.seed, kind=c.content)[0]
     om = oracle.build(oracle.ModemSpec(c.kind, c.variant, c.width, c.height, c.standard, c.chroma_avg, c.notch, c.opt))
     return g, rgb, om

@@ -1,19 +1,11 @@
 """CPU: the oracle reproduces every golden fixture generated from the reference itself (tests/golden/make_golden.py)."""
-import os
-
 import numpy as np
 import pytest
 
 import oracle
 from oracle import frame as oframe
-from cases import GOLDEN_CASES, FLOAT_ROWS, case_id
+from cases import GOLDEN_CASES, FLOAT_ROWS, case_id, load_golden
 from color_modem_b200.synth import synth_frames_u8
-
-GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
-
-
-def load_golden(c):
-    return np.load(os.path.join(GOLDEN_DIR, case_id(c) + '.npz'))
 
 
 @pytest.mark.parametrize('c', GOLDEN_CASES, ids=case_id)

@@ -1,5 +1,5 @@
-"""Builder-container only: re-check the oracle against the live reference at full frame size.
-Skipped wherever /root/reference is absent (e.g. the GPU box)."""
+"""CPU: the oracle at full frame size (BASELINE configs 1-5) against the stored frames of tests/golden/full-*.npz, byte for
+byte; where COLOR_MODEM_REFERENCE names a checkout of the reference (tests/refload.py), also against the live reference."""
 import warnings
 
 import numpy as np
@@ -7,33 +7,32 @@ import pytest
 
 import oracle
 from oracle import frame as oframe
-from cases import Case
+from cases import FULL_CASES, frame_digest, load_full
 from refload import reference_available, load_reference
 from color_modem_b200.synth import synth_frames_u8
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not reference_available(), reason='/root/reference not present')]
 
-FULL = [
-    Case('ntsc', 'NTSC', 720, 480, None, False, 0, 0, 'smooth'),          # BASELINE config 1
-    Case('pal_d', 'PAL', 720, 576, None, False, 0, 0, 'smooth'),          # BASELINE config 2
-    Case('ntsc_3d', 'NTSC', 720, 480, None, False, 599, 3, 'smooth'),     # BASELINE config 3 (last frame)
-    Case('secam', 'SECAM', 720, 576, None, True, 7, 4, 'noise'),          # BASELINE config 4a
-    Case('niir_hue', 'PAL', 720, 576, None, False, 999, 5, 'smooth'),     # BASELINE config 4b
-    Case('mac', 'D2MAC_7MHZ', 1920, 1080, 'GERBER_625', False, 2, 6, 'smooth'),   # BASELINE config 5 sample
-]
+def _assert_stored(frame, g, name):
+    assert frame.shape == tuple(g[name + '_shape'])
+    diff = np.nonzero((frame[g['rows']] != g[name + '_rows']).reshape(len(g['rows']), -1).any(axis=1))[0]
+    assert not len(diff), '%s differs from the %s frame on rows %s' % (name, g['source'], g['rows'][diff])
+    assert np.array_equal(frame_digest(frame), g[name + '_sha256']), '%s differs from the %s frame' % (name, g['source'])
 
 
-@pytest.mark.parametrize('c', FULL, ids=lambda c: '%s-%s-%dx%d' % (c.kind, c.variant, c.width, c.height))
+@pytest.mark.parametrize('c', FULL_CASES, ids=lambda c: '%s-%s-%dx%d' % (c.kind, c.variant, c.width, c.height))
 def test_full_frame_u8_identical(c):
-    warnings.filterwarnings('ignore')
-    from PIL import Image
-    ref = load_reference()
     rgb = synth_frames_u8(1, c.height, c.width, first_frame=c.frame, seed=c.seed, kind=c.content)[0]
-    driver = ref.image.ImageModem(ref.make_modem(c))
-    comp_img = driver.modulate(Image.fromarray(rgb, 'RGB'), c.frame)
-    comp_ref = np.asarray(comp_img)
-    out_ref = np.asarray(driver.demodulate(comp_img, c.frame))
     modem = oracle.build(oracle.ModemSpec(c.kind, c.variant, c.width, c.height, c.standard, c.chroma_avg, c.notch, c.opt))
-    assert np.array_equal(oframe.encode_frame_u8(modem, c.frame, rgb), comp_ref)
-    assert np.array_equal(oframe.decode_frame_u8(modem, c.frame, comp_ref), out_ref)
+    comp = oframe.encode_frame_u8(modem, c.frame, rgb)
+    g = load_full(c)
+    _assert_stored(comp, g, 'comp')
+    out = oframe.decode_frame_u8(modem, c.frame, comp)
+    _assert_stored(out, g, 'rgb')
+    if reference_available():
+        warnings.filterwarnings('ignore')
+        from PIL import Image
+        ref = load_reference()
+        driver = ref.image.ImageModem(ref.make_modem(c))
+        comp_img = driver.modulate(Image.fromarray(rgb, 'RGB'), c.frame)
+        assert np.array_equal(comp, np.asarray(comp_img))
+        assert np.array_equal(out, np.asarray(driver.demodulate(comp_img, c.frame)))
