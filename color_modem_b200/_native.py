@@ -58,9 +58,20 @@ class Window(C.Structure):
 MODE_DEFAULT, MODE_BANDSPLIT_NOSTRIP, MODE_EXTRACT_CHROMA = 0, 1, 2
 
 
+class PixFmt(C.Structure):
+    _fields_ = [('format', C.c_int32), ('matrix', C.c_int32), ('range', C.c_int32), ('reserved', C.c_int32)]
+
+
+PIX_RGB24, PIX_YUV420P = 0, 1
+YUV_BT601, YUV_BT709 = 0, 1
+YUV_LIMITED, YUV_FULL = 0, 1
+
+
 EXPORTS = ['cm_abi_version', 'cm_sizeof_desc', 'cm_last_error', 'cm_device_info', 'cm_create', 'cm_destroy', 'cm_encode_frames',
            'cm_decode_frames', 'cm_encode_ex', 'cm_decode_ex', 'cm_encode_frames_host', 'cm_decode_frames_host',
-           'cm_filter_rows', 'cm_transcode_frames_host', 'cm_measure_fma_peak', 'cm_launch_count', 'cm_timing_enable', 'cm_timing_reset', 'cm_timing_read', 'cm_phase_profile']
+           'cm_filter_rows', 'cm_transcode_frames_host', 'cm_measure_fma_peak', 'cm_launch_count', 'cm_timing_enable', 'cm_timing_reset', 'cm_timing_read', 'cm_phase_profile',
+           'cm_yuv420p_to_rgb24', 'cm_rgb24_to_yuv420p', 'cm_encode_frames_host_fmt', 'cm_decode_frames_host_fmt',
+           'cm_transcode_frames_host_fmt']
 
 K_ENCODE, K_BANDSPLIT, K_PALD, K_COMB, K_DECODE_OTHER = 0, 1, 2, 3, 4
 
@@ -93,6 +104,12 @@ def load():
     lib.cm_encode_frames_host.argtypes = [vp, vp, vp, i64, i32]
     lib.cm_decode_frames_host.argtypes = [vp, vp, vp, i64, i32]
     lib.cm_transcode_frames_host.argtypes = [vp, vp, vp, vp, i64, i32]
+    pf = C.POINTER(PixFmt)
+    lib.cm_yuv420p_to_rgb24.argtypes = [pf, vp, vp, i32, i32, i32, vp]
+    lib.cm_rgb24_to_yuv420p.argtypes = [pf, vp, vp, i32, i32, i32, vp]
+    lib.cm_encode_frames_host_fmt.argtypes = [vp, vp, vp, i64, i32, pf]
+    lib.cm_decode_frames_host_fmt.argtypes = [vp, vp, vp, i64, i32, pf]
+    lib.cm_transcode_frames_host_fmt.argtypes = [vp, vp, vp, vp, i64, i32, pf]
     lib.cm_measure_fma_peak.argtypes = [C.POINTER(C.c_double)]
     lib.cm_filter_rows.argtypes = [C.POINTER(Filter), C.c_int, vp, vp, i32, vp]
     lib.cm_launch_count.restype = C.c_int64

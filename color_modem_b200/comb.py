@@ -193,27 +193,34 @@ class SimpleCombModem(_Fused):
     def encode_frames(self, rgb, first_frame=0, out=None, out_float=None):
         return (self._impl or self.backend).encode_frames(rgb, first_frame, out=out, out_float=out_float)
 
-    def encode_frames_host(self, rgb, first_frame=0, out=None):
-        return (self._impl or self.backend).encode_frames_host(rgb, first_frame, out=out)
+    def encode_frames_host(self, rgb, first_frame=0, out=None, pix_fmt=None):
+        return (self._impl or self.backend).encode_frames_host(rgb, first_frame, out=out, pix_fmt=pix_fmt)
 
-    def decode_frames_host(self, comp, first_frame=0, out=None):
+    def decode_frames_host(self, comp, first_frame=0, out=None, pix_fmt=None):
         if self._impl is not None:
-            return self._impl.decode_frames_host(comp, first_frame, out=out)
+            return self._impl.decode_frames_host(comp, first_frame, out=out, pix_fmt=pix_fmt)
         from .image import drive_demodulate_u8
+        from .pixfmt import from_rgb24, frame_shape, resolve
+        fmt = resolve(pix_fmt)
         comp = numpy.ascontiguousarray(comp, dtype=numpy.uint8)
         res = numpy.stack([drive_demodulate_u8(self, comp[i], first_frame + i) for i in range(comp.shape[0])]) \
             if comp.shape[0] else numpy.empty((0, comp.shape[1], self.backend.output_width, 3), numpy.uint8)
+        if not fmt.is_rgb24:          # the composed path is u8 RGB; the conversion runs on the device around it
+            import torch
+            res = from_rgb24(torch.from_numpy(res).cuda(), fmt).cpu().numpy() if res.shape[0] else \
+                numpy.empty((0,) + frame_shape(fmt, self.backend.output_width, comp.shape[1]), numpy.uint8)
         if out is not None:
             out[...] = res
             return out
         return res
 
-    def transcode_frames_host(self, rgb, first_frame=0, out=None, comp_out=None, want_composite=True):
+    def transcode_frames_host(self, rgb, first_frame=0, out=None, comp_out=None, want_composite=True, pix_fmt=None):
         if self._impl is not None:
             return self._impl.transcode_frames_host(rgb, first_frame, out=out, comp_out=comp_out,
-                                                    want_composite=want_composite)
-        comp = self.encode_frames_host(rgb, first_frame, out=comp_out)
-        return (comp if want_composite or comp_out is not None else None), self.decode_frames_host(comp, first_frame, out=out)
+                                                    want_composite=want_composite, pix_fmt=pix_fmt)
+        comp = self.encode_frames_host(rgb, first_frame, out=comp_out, pix_fmt=pix_fmt)
+        return (comp if want_composite or comp_out is not None else None), \
+            self.decode_frames_host(comp, first_frame, out=out, pix_fmt=pix_fmt)
 
     def decode_frames(self, comp, first_frame=0, out=None, out_float=None):
         if self._impl is not None:

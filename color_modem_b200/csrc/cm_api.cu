@@ -600,6 +600,7 @@ extern "C" void cm_destroy(cm_modem *m) {
         cudaFree(m->d_in[i]);
         cudaFree(m->d_out[i]);
         cudaFree(m->d_mid[i]);
+        cudaFree(m->d_rgb[i]);
         if (m->ev_in[i]) cudaEventDestroy(m->ev_in[i]);
         if (m->ev_k[i]) cudaEventDestroy(m->ev_k[i]);
         if (m->ev_mid[i]) cudaEventDestroy(m->ev_mid[i]);
@@ -825,12 +826,17 @@ static int ensure(void **buf, size_t *cap, size_t need) {
 // concurrently (two copy engines + SMs); with pageable memory it is still correct, just serialised by the driver.
 // what: 0 encode (in = RGB, out = composite), 1 decode (in = composite, out = RGB), 2 encode -> decode with the composite
 // staying in device memory (in = RGB, out = RGB, mid = composite copy-out or null).
+// f: picture format of the RGB side (NULL = rgb24).  For yuv420p only the 4:2:0 frames cross the link: the conversion to
+// RGB runs on the kernel stream before the encoder and the one back after the decoder, through one device RGB buffer per
+// staging slot; in_frame / out_frame are the link-side frame sizes.
 static int run_host(cm_modem *m, int what, const uint8_t *in, uint8_t *out, uint8_t *mid, size_t in_frame, size_t out_frame,
-                    size_t mid_frame, int64_t first_frame, int32_t nframes) {
+                    size_t mid_frame, int64_t first_frame, int32_t nframes, const cm_pixfmt *f) {
     if (!m || !in || !out) return fail(CM_ERR_INVALID, "null argument%s");
     if (nframes < 0) return fail(CM_ERR_INVALID, "bad frame count%s");
     if (nframes == 0) return CM_OK;
     CUDA_TRY(cudaSetDevice(m->device));
+    const bool yuv = f && f->format == CM_PIX_YUV420P;
+    const int W = m->desc.width, H = m->desc.height, Wo = m->desc.out_width;
     int chunk = m->tune.host_chunk;
     if (chunk > nframes) chunk = nframes;
     for (int s = 0; s < cm_modem::kHostStreams; ++s)
@@ -841,6 +847,7 @@ static int run_host(cm_modem *m, int what, const uint8_t *in, uint8_t *out, uint
         int rc = ensure(&m->d_in[b], &m->in_cap[b], (size_t)chunk * in_frame);
         if (!rc) rc = ensure(&m->d_out[b], &m->out_cap[b], (size_t)chunk * out_frame);
         if (!rc && what == 2) rc = ensure(&m->d_mid[b], &m->mid_cap[b], (size_t)chunk * mid_frame);
+        if (!rc && yuv) rc = ensure(&m->d_rgb[b], &m->rgb_cap[b], (size_t)chunk * H * (W > Wo ? W : Wo) * 3);
         if (rc) return rc;
         if (!m->ev_in[b]) {
             CUDA_TRY(cudaEventCreateWithFlags(&m->ev_in[b], cudaEventDisableTiming));
@@ -849,6 +856,16 @@ static int run_host(cm_modem *m, int what, const uint8_t *in, uint8_t *out, uint
             CUDA_TRY(cudaEventCreateWithFlags(&m->ev_out[b], cudaEventDisableTiming));
         }
     }
+    // RGB frames the encoder reads / the decoder writes: the staging buffers themselves for rgb24, d_rgb[b] for yuv420p
+    auto to_rgb = [&](const uint8_t *din, uint8_t *drgb, int n, cudaStream_t st, const uint8_t **pin) -> int {
+        *pin = din;
+        if (!yuv || what == 1) return CM_OK;
+        *pin = drgb;
+        return cm_yuv420p_to_rgb24(f, din, drgb, W, H, n, st);
+    };
+    auto from_rgb = [&](const uint8_t *drgb, uint8_t *dout, int n, cudaStream_t st) -> int {
+        return yuv && what != 0 ? cm_rgb24_to_yuv420p(f, drgb, dout, Wo, H, n, st) : (int)CM_OK;
+    };
     if (roles) {
         // One stream per role: every host->device copy on hs[0], every kernel on hs[1], every device->host copy on hs[2],
         // chained per staging buffer by events.  (With one stream per chunk the copy-in of chunk i + 3 queued behind the
@@ -856,37 +873,40 @@ static int run_host(cm_modem *m, int what, const uint8_t *in, uint8_t *out, uint
         cudaStream_t s_in = m->hs[0], s_k = m->hs[1], s_out = m->hs[2];
         int rc = CM_OK;
         cudaError_t ce = cudaSuccess;
-        for (int f = 0, i = 0; f < nframes && rc == CM_OK && ce == cudaSuccess; f += chunk, ++i) {
+        for (int f0 = 0, i = 0; f0 < nframes && rc == CM_OK && ce == cudaSuccess; f0 += chunk, ++i) {
             const int b = i % nbuf;
-            const int n = nframes - f < chunk ? nframes - f : chunk;
-            const uint8_t *din = (const uint8_t *)m->d_in[b];
-            uint8_t *dout = (uint8_t *)m->d_out[b], *dmid = (uint8_t *)m->d_mid[b];
+            const int n = nframes - f0 < chunk ? nframes - f0 : chunk;
+            const uint8_t *din = (const uint8_t *)m->d_in[b], *pin = din;
+            uint8_t *dout = (uint8_t *)m->d_out[b], *dmid = (uint8_t *)m->d_mid[b], *drgb = (uint8_t *)m->d_rgb[b];
+            uint8_t *pout = yuv ? drgb : dout;
             if (i >= nbuf) ce = cudaStreamWaitEvent(s_in, m->ev_k[b], 0);             // the kernels of chunk i - nbuf have read d_in[b]
             if (ce == cudaSuccess)
-                ce = cudaMemcpyAsync(m->d_in[b], in + (size_t)f * in_frame, (size_t)n * in_frame, cudaMemcpyHostToDevice, s_in);
+                ce = cudaMemcpyAsync(m->d_in[b], in + (size_t)f0 * in_frame, (size_t)n * in_frame, cudaMemcpyHostToDevice, s_in);
             if (ce == cudaSuccess) ce = cudaEventRecord(m->ev_in[b], s_in);
             if (ce == cudaSuccess) ce = cudaStreamWaitEvent(s_k, m->ev_in[b], 0);
             if (ce == cudaSuccess && i >= nbuf) ce = cudaStreamWaitEvent(s_k, m->ev_out[b], 0);   // d_out[b] / d_mid[b] copied out
             if (ce != cudaSuccess) break;
             m->aux_slot = 1;                                                          // one kernel stream: one scratch
-            if (what == 0) rc = cm_encode_frames(m, din, dout, first_frame + f, n, s_k);
-            else if (what == 1) rc = cm_decode_frames(m, din, dout, first_frame + f, n, s_k);
-            else {
-                rc = cm_encode_frames(m, din, dmid, first_frame + f, n, s_k);
+            rc = to_rgb(din, drgb, n, s_k, &pin);
+            if (rc == CM_OK && what == 0) rc = cm_encode_frames(m, pin, dout, first_frame + f0, n, s_k);
+            else if (rc == CM_OK && what == 1) rc = cm_decode_frames(m, din, pout, first_frame + f0, n, s_k);
+            else if (rc == CM_OK) {
+                rc = cm_encode_frames(m, pin, dmid, first_frame + f0, n, s_k);
                 if (rc == CM_OK && mid) {
                     ce = cudaEventRecord(m->ev_mid[b], s_k);
                     if (ce == cudaSuccess) ce = cudaStreamWaitEvent(s_out, m->ev_mid[b], 0);
                     if (ce == cudaSuccess)
-                        ce = cudaMemcpyAsync(mid + (size_t)f * mid_frame, dmid, (size_t)n * mid_frame, cudaMemcpyDeviceToHost, s_out);
+                        ce = cudaMemcpyAsync(mid + (size_t)f0 * mid_frame, dmid, (size_t)n * mid_frame, cudaMemcpyDeviceToHost, s_out);
                 }
-                if (rc == CM_OK && ce == cudaSuccess) rc = cm_decode_frames(m, dmid, dout, first_frame + f, n, s_k);
+                if (rc == CM_OK && ce == cudaSuccess) rc = cm_decode_frames(m, dmid, pout, first_frame + f0, n, s_k);
             }
+            if (rc == CM_OK && ce == cudaSuccess) rc = from_rgb(drgb, dout, n, s_k);
             m->aux_slot = 0;
             if (rc != CM_OK || ce != cudaSuccess) break;
             ce = cudaEventRecord(m->ev_k[b], s_k);
             if (ce == cudaSuccess) ce = cudaStreamWaitEvent(s_out, m->ev_k[b], 0);
             if (ce == cudaSuccess)
-                ce = cudaMemcpyAsync(out + (size_t)f * out_frame, dout, (size_t)n * out_frame, cudaMemcpyDeviceToHost, s_out);
+                ce = cudaMemcpyAsync(out + (size_t)f0 * out_frame, dout, (size_t)n * out_frame, cudaMemcpyDeviceToHost, s_out);
             if (ce == cudaSuccess) ce = cudaEventRecord(m->ev_out[b], s_out);
         }
         // also on failure: no copy into the caller's memory may still be in flight when this returns
@@ -900,26 +920,29 @@ static int run_host(cm_modem *m, int what, const uint8_t *in, uint8_t *out, uint
     }
     int rc = CM_OK;
     cudaError_t ce = cudaSuccess;
-    for (int f = 0, i = 0; f < nframes && rc == CM_OK && ce == cudaSuccess; f += chunk, ++i) {
+    for (int f0 = 0, i = 0; f0 < nframes && rc == CM_OK && ce == cudaSuccess; f0 += chunk, ++i) {
         const int s = i % cm_modem::kHostStreams;
-        const int n = nframes - f < chunk ? nframes - f : chunk;
+        const int n = nframes - f0 < chunk ? nframes - f0 : chunk;
         cudaStream_t st = m->hs[s];
-        ce = cudaMemcpyAsync(m->d_in[s], in + (size_t)f * in_frame, (size_t)n * in_frame, cudaMemcpyHostToDevice, st);
+        ce = cudaMemcpyAsync(m->d_in[s], in + (size_t)f0 * in_frame, (size_t)n * in_frame, cudaMemcpyHostToDevice, st);
         if (ce != cudaSuccess) break;
         m->aux_slot = 1 + s;
-        const uint8_t *din = (const uint8_t *)m->d_in[s];
-        uint8_t *dout = (uint8_t *)m->d_out[s], *dmid = (uint8_t *)m->d_mid[s];
-        if (what == 0) rc = cm_encode_frames(m, din, dout, first_frame + f, n, st);
-        else if (what == 1) rc = cm_decode_frames(m, din, dout, first_frame + f, n, st);
-        else {
-            rc = cm_encode_frames(m, din, dmid, first_frame + f, n, st);
+        const uint8_t *din = (const uint8_t *)m->d_in[s], *pin = din;
+        uint8_t *dout = (uint8_t *)m->d_out[s], *dmid = (uint8_t *)m->d_mid[s], *drgb = (uint8_t *)m->d_rgb[s];
+        uint8_t *pout = yuv ? drgb : dout;
+        rc = to_rgb(din, drgb, n, st, &pin);
+        if (rc == CM_OK && what == 0) rc = cm_encode_frames(m, pin, dout, first_frame + f0, n, st);
+        else if (rc == CM_OK && what == 1) rc = cm_decode_frames(m, din, pout, first_frame + f0, n, st);
+        else if (rc == CM_OK) {
+            rc = cm_encode_frames(m, pin, dmid, first_frame + f0, n, st);
             if (rc == CM_OK && mid)
-                ce = cudaMemcpyAsync(mid + (size_t)f * mid_frame, dmid, (size_t)n * mid_frame, cudaMemcpyDeviceToHost, st);
-            if (rc == CM_OK) rc = cm_decode_frames(m, dmid, dout, first_frame + f, n, st);
+                ce = cudaMemcpyAsync(mid + (size_t)f0 * mid_frame, dmid, (size_t)n * mid_frame, cudaMemcpyDeviceToHost, st);
+            if (rc == CM_OK) rc = cm_decode_frames(m, dmid, pout, first_frame + f0, n, st);
         }
+        if (rc == CM_OK && ce == cudaSuccess) rc = from_rgb(drgb, dout, n, st);
         m->aux_slot = 0;
         if (rc == CM_OK && ce == cudaSuccess)
-            ce = cudaMemcpyAsync(out + (size_t)f * out_frame, dout, (size_t)n * out_frame, cudaMemcpyDeviceToHost, st);
+            ce = cudaMemcpyAsync(out + (size_t)f0 * out_frame, dout, (size_t)n * out_frame, cudaMemcpyDeviceToHost, st);
     }
     // also on failure: no copy into the caller's memory may still be in flight when this returns
     for (int s = 0; s < cm_modem::kHostStreams; ++s) {
@@ -931,24 +954,53 @@ static int run_host(cm_modem *m, int what, const uint8_t *in, uint8_t *out, uint
     return CM_OK;
 }
 
+// Bytes of one picture-side frame w wide in format f (NULL = rgb24); 0 for a format that does not exist.
+static size_t pic_frame(const cm_pixfmt *f, int w, int h) {
+    if (!f || f->format == CM_PIX_RGB24) return (size_t)h * w * 3;
+    if (f->format != CM_PIX_YUV420P || f->reserved || (f->matrix != CM_YUV_BT601 && f->matrix != CM_YUV_BT709) ||
+        (f->range != CM_YUV_LIMITED && f->range != CM_YUV_FULL))
+        return 0;
+    return (size_t)h * w + (size_t)w * ((h + 1) / 2);        // Y + U + V: W H + 2 (W/2) ceil(H/2)
+}
+
+extern "C" int cm_encode_frames_host_fmt(cm_modem *m, const uint8_t *pic, uint8_t *comp, int64_t first_frame,
+                                         int32_t nframes, const cm_pixfmt *f) {
+    if (!m) return fail(CM_ERR_INVALID, "null handle%s");
+    const size_t in_frame = pic_frame(f, m->desc.width, m->desc.height);
+    if (!in_frame) return fail(CM_ERR_INVALID, "bad cm_pixfmt%s");
+    return run_host(m, 0, pic, comp, nullptr, in_frame, (size_t)m->desc.height * m->desc.comp_width, 0, first_frame, nframes,
+                    f);
+}
+
+extern "C" int cm_decode_frames_host_fmt(cm_modem *m, const uint8_t *comp, uint8_t *pic, int64_t first_frame,
+                                         int32_t nframes, const cm_pixfmt *f) {
+    if (!m) return fail(CM_ERR_INVALID, "null handle%s");
+    const size_t out_frame = pic_frame(f, m->desc.out_width, m->desc.height);
+    if (!out_frame) return fail(CM_ERR_INVALID, "bad cm_pixfmt%s");
+    return run_host(m, 1, comp, pic, nullptr, (size_t)m->desc.height * m->desc.comp_width, out_frame, 0, first_frame, nframes,
+                    f);
+}
+
+extern "C" int cm_transcode_frames_host_fmt(cm_modem *m, const uint8_t *pic_in, uint8_t *comp_out, uint8_t *pic_out,
+                                            int64_t first_frame, int32_t nframes, const cm_pixfmt *f) {
+    if (!m) return fail(CM_ERR_INVALID, "null handle%s");
+    const size_t in_frame = pic_frame(f, m->desc.width, m->desc.height), out_frame = pic_frame(f, m->desc.out_width, m->desc.height);
+    if (!in_frame) return fail(CM_ERR_INVALID, "bad cm_pixfmt%s");
+    return run_host(m, 2, pic_in, pic_out, comp_out, in_frame, out_frame, (size_t)m->desc.height * m->desc.comp_width,
+                    first_frame, nframes, f);
+}
+
 extern "C" int cm_encode_frames_host(cm_modem *m, const uint8_t *rgb, uint8_t *comp, int64_t first_frame,
                                      int32_t nframes) {
-    if (!m) return fail(CM_ERR_INVALID, "null handle%s");
-    return run_host(m, 0, rgb, comp, nullptr, (size_t)m->desc.height * m->desc.width * 3,
-                    (size_t)m->desc.height * m->desc.comp_width, 0, first_frame, nframes);
+    return cm_encode_frames_host_fmt(m, rgb, comp, first_frame, nframes, nullptr);
 }
 
 extern "C" int cm_decode_frames_host(cm_modem *m, const uint8_t *comp, uint8_t *rgb, int64_t first_frame,
                                      int32_t nframes) {
-    if (!m) return fail(CM_ERR_INVALID, "null handle%s");
-    return run_host(m, 1, comp, rgb, nullptr, (size_t)m->desc.height * m->desc.comp_width,
-                    (size_t)m->desc.height * m->desc.out_width * 3, 0, first_frame, nframes);
+    return cm_decode_frames_host_fmt(m, comp, rgb, first_frame, nframes, nullptr);
 }
 
 extern "C" int cm_transcode_frames_host(cm_modem *m, const uint8_t *rgb_in, uint8_t *comp_out, uint8_t *rgb_out,
                                         int64_t first_frame, int32_t nframes) {
-    if (!m) return fail(CM_ERR_INVALID, "null handle%s");
-    return run_host(m, 2, rgb_in, rgb_out, comp_out, (size_t)m->desc.height * m->desc.width * 3,
-                    (size_t)m->desc.height * m->desc.out_width * 3, (size_t)m->desc.height * m->desc.comp_width, first_frame,
-                    nframes);
+    return cm_transcode_frames_host_fmt(m, rgb_in, comp_out, rgb_out, first_frame, nframes, nullptr);
 }

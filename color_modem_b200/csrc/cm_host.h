@@ -76,7 +76,8 @@ struct cm_modem {
     cudaStream_t hs[kHostStreams] = {nullptr, nullptr, nullptr};
     void *d_in[kHostBufs] = {}, *d_out[kHostBufs] = {};
     void *d_mid[kHostBufs] = {};                // cm_transcode_frames_host: the composite between the two halves
-    size_t in_cap[kHostBufs] = {}, out_cap[kHostBufs] = {}, mid_cap[kHostBufs] = {};
+    void *d_rgb[kHostBufs] = {};                // *_host_fmt with yuv420p: the RGB frames beside the link-side staging
+    size_t in_cap[kHostBufs] = {}, out_cap[kHostBufs] = {}, mid_cap[kHostBufs] = {}, rgb_cap[kHostBufs] = {};
     cudaEvent_t ev_in[kHostBufs] = {}, ev_k[kHostBufs] = {}, ev_mid[kHostBufs] = {}, ev_out[kHostBufs] = {};
 };
 

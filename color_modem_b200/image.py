@@ -49,17 +49,20 @@ class ImageModem(object):
     def decode_composite_level(value):
         return (5.0 * value - 1.0) / 3.0
 
-    def modulate_batch(self, rgb_u8, first_frame=0, out=None):
-        return self._modem.encode_frames_host(rgb_u8, first_frame, out=out)
+    def modulate_batch(self, rgb_u8, first_frame=0, out=None, pix_fmt=None):
+        """[N, H, W, 3] rgb24 frames (or, with ``pix_fmt`` a yuv420p PixelFormat, [N, frame_bytes]) -> [N, H, Wc] composite."""
+        return self._modem.encode_frames_host(rgb_u8, first_frame, out=out, pix_fmt=pix_fmt)
 
-    def demodulate_batch(self, comp_u8, first_frame=0, out=None):
-        return self._modem.decode_frames_host(comp_u8, first_frame, out=out)
+    def demodulate_batch(self, comp_u8, first_frame=0, out=None, pix_fmt=None):
+        """[N, H, Wc] composite -> [N, H, Wo, 3] rgb24 frames (or [N, frame_bytes] yuv420p, ``output_width`` wide)."""
+        return self._modem.decode_frames_host(comp_u8, first_frame, out=out, pix_fmt=pix_fmt)
 
-    def transcode_batch(self, rgb_u8, first_frame=0, out=None, comp_out=None, want_composite=True):
+    def transcode_batch(self, rgb_u8, first_frame=0, out=None, comp_out=None, want_composite=True, pix_fmt=None):
         """modulate_batch then demodulate_batch of the result in one native call: the composite is handed over in device
-        memory (and copied out too unless ``want_composite`` is false).  Returns (composite or None, rgb)."""
+        memory (and copied out too unless ``want_composite`` is false).  Returns (composite or None, rgb).  With ``pix_fmt``
+        yuv420p only the 4:2:0 frames cross the host link; the conversions run on the GPU."""
         return self._modem.transcode_frames_host(rgb_u8, first_frame, out=out, comp_out=comp_out,
-                                                 want_composite=want_composite)
+                                                 want_composite=want_composite, pix_fmt=pix_fmt)
 
     def modulate(self, img, frame=0):
         from PIL import Image

@@ -176,36 +176,62 @@ class GpuModem(object):
             raise ValueError('out must be a C-contiguous uint8 array of shape %s' % (shape,))
         return out
 
-    def encode_frames_host(self, rgb, first_frame=0, out=None):
-        rgb = numpy.ascontiguousarray(rgb, dtype=numpy.uint8)
-        if rgb.shape[1:] != (self.height, self.width, 3):
-            raise ValueError('expected uint8 [N, %d, %d, 3]' % (self.height, self.width))
+    def _pic_in(self, pic, fmt, w):
+        """Picture-side input batch: rgb24 [N, H, w, 3] or yuv420p [N, frame_bytes]."""
+        from .pixfmt import frame_shape
+        shape = frame_shape(fmt, w, self.height)
+        pic = numpy.ascontiguousarray(pic, dtype=numpy.uint8)
+        if pic.shape[1:] != shape:
+            raise ValueError('expected %s uint8 [N, %s]' % (fmt.name, ', '.join(map(str, shape))))
+        return pic
+
+    def encode_frames_host(self, rgb, first_frame=0, out=None, pix_fmt=None):
+        """rgb24 [N, H, W, 3] (or, with ``pix_fmt`` yuv420p, [N, frame_bytes]) host frames -> composite [N, H, Wc]."""
+        from .pixfmt import resolve
+        fmt = resolve(pix_fmt)
+        rgb = self._pic_in(rgb, fmt, self.width)
         out = self._host_out(out, (rgb.shape[0], self.height, self.composite_width))
-        N.check(N.load().cm_encode_frames_host(self._handle(), rgb.ctypes.data, out.ctypes.data, int(first_frame),
-                                               int(rgb.shape[0])))
+        if fmt.is_rgb24:
+            N.check(N.load().cm_encode_frames_host(self._handle(), rgb.ctypes.data, out.ctypes.data, int(first_frame),
+                                                   int(rgb.shape[0])))
+        else:
+            N.check(N.load().cm_encode_frames_host_fmt(self._handle(), rgb.ctypes.data, out.ctypes.data, int(first_frame),
+                                                       int(rgb.shape[0]), C.byref(fmt.c_struct())))
         return out
 
-    def decode_frames_host(self, comp, first_frame=0, out=None):
+    def decode_frames_host(self, comp, first_frame=0, out=None, pix_fmt=None):
+        """composite [N, H, Wc] -> rgb24 [N, H, Wo, 3] (or, with ``pix_fmt`` yuv420p, [N, frame_bytes of Wo x H])."""
+        from .pixfmt import frame_shape, resolve
+        fmt = resolve(pix_fmt)
         comp = numpy.ascontiguousarray(comp, dtype=numpy.uint8)
         if comp.shape[1:] != (self.height, self.composite_width):
             raise ValueError('expected uint8 [N, %d, %d]' % (self.height, self.composite_width))
-        out = self._host_out(out, (comp.shape[0], self.height, self.output_width, 3))
-        N.check(N.load().cm_decode_frames_host(self._handle(), comp.ctypes.data, out.ctypes.data, int(first_frame),
-                                               int(comp.shape[0])))
+        out = self._host_out(out, (comp.shape[0],) + frame_shape(fmt, self.output_width, self.height))
+        if fmt.is_rgb24:
+            N.check(N.load().cm_decode_frames_host(self._handle(), comp.ctypes.data, out.ctypes.data, int(first_frame),
+                                                   int(comp.shape[0])))
+        else:
+            N.check(N.load().cm_decode_frames_host_fmt(self._handle(), comp.ctypes.data, out.ctypes.data, int(first_frame),
+                                                       int(comp.shape[0]), C.byref(fmt.c_struct())))
         return out
 
-    def transcode_frames_host(self, rgb, first_frame=0, out=None, comp_out=None, want_composite=True):
+    def transcode_frames_host(self, rgb, first_frame=0, out=None, comp_out=None, want_composite=True, pix_fmt=None):
         """encode_frames_host followed by decode_frames_host of its result (what the reference's cli.py:62-65 does), the
-        composite staying in device memory between the two.  Returns (composite or None, rgb)."""
-        rgb = numpy.ascontiguousarray(rgb, dtype=numpy.uint8)
-        if rgb.shape[1:] != (self.height, self.width, 3):
-            raise ValueError('expected uint8 [N, %d, %d, 3]' % (self.height, self.width))
-        out = self._host_out(out, (rgb.shape[0], self.height, self.output_width, 3))
+        composite staying in device memory between the two.  Returns (composite or None, rgb).  With ``pix_fmt`` yuv420p
+        both picture sides are yuv420p frames (the output ``output_width`` wide)."""
+        from .pixfmt import frame_shape, resolve
+        fmt = resolve(pix_fmt)
+        rgb = self._pic_in(rgb, fmt, self.width)
+        out = self._host_out(out, (rgb.shape[0],) + frame_shape(fmt, self.output_width, self.height))
         if want_composite or comp_out is not None:
             comp_out = self._host_out(comp_out, (rgb.shape[0], self.height, self.composite_width))
-        N.check(N.load().cm_transcode_frames_host(self._handle(), rgb.ctypes.data,
-                                                  comp_out.ctypes.data if comp_out is not None else None,
-                                                  out.ctypes.data, int(first_frame), int(rgb.shape[0])))
+        comp_ptr = comp_out.ctypes.data if comp_out is not None else None
+        if fmt.is_rgb24:
+            N.check(N.load().cm_transcode_frames_host(self._handle(), rgb.ctypes.data, comp_ptr, out.ctypes.data,
+                                                      int(first_frame), int(rgb.shape[0])))
+        else:
+            N.check(N.load().cm_transcode_frames_host_fmt(self._handle(), rgb.ctypes.data, comp_ptr, out.ctypes.data,
+                                                          int(first_frame), int(rgb.shape[0]), C.byref(fmt.c_struct())))
         return comp_out, out
 
     # ---- float frames (parity tests: composite before the level map / RGB before clipping) -------------------

@@ -197,6 +197,37 @@ int cm_decode_frames_host(cm_modem *m, const uint8_t *comp, uint8_t *rgb, int64_
 int cm_transcode_frames_host(cm_modem *m, const uint8_t *rgb_in, uint8_t *comp_out, uint8_t *rgb_out, int64_t first_frame,
                              int32_t nframes);
 
+/* Picture format of the frame-batch paths.  CM_PIX_RGB24: packed [H][W][3] bytes, the format of every call above.
+ * CM_PIX_YUV420P: planar 8-bit YUV 4:2:0 (I420): Y [H][W], then U (Cb) [ceil(H/2)][W/2], then V (Cr) [ceil(H/2)][W/2];
+ * W * H + 2 * (W/2) * ceil(H/2) bytes per frame; chroma rows are 2-byte aligned only.  `matrix` and `range` select the
+ * colour matrix (BT.601: Kr 0.299, Kb 0.114; BT.709: Kr 0.2126, Kb 0.0722) and the quantisation (limited: Y' 16..235,
+ * C 16..240; full: 0..255).  The conversion is exact integer arithmetic in Q16 (INTEGRATION.md, "Picture formats"):
+ * RGB -> YUV averages each 2x2 chroma block (an odd height's last row counts twice), YUV -> RGB upsamples the chroma by
+ * nearest neighbour.  `reserved` must be 0. */
+enum cm_pix_format { CM_PIX_RGB24 = 0, CM_PIX_YUV420P = 1 };
+enum cm_yuv_matrix { CM_YUV_BT601 = 0, CM_YUV_BT709 = 1 };
+enum cm_yuv_range { CM_YUV_LIMITED = 0, CM_YUV_FULL = 1 };
+typedef struct cm_pixfmt {
+    int32_t format, matrix, range, reserved;
+} cm_pixfmt;
+
+/* Device conversions between yuv420p [n][frame bytes] and rgb24 [n][H][W][3] (DEVICE pointers).  f->format must be
+ * CM_PIX_YUV420P; width a multiple of 4.  Stream-ordered, allocate nothing, may be captured in a CUDA graph. */
+int cm_yuv420p_to_rgb24(const cm_pixfmt *f, const uint8_t *yuv, uint8_t *rgb, int32_t width, int32_t height, int32_t nframes,
+                        void *stream);
+int cm_rgb24_to_yuv420p(const cm_pixfmt *f, const uint8_t *rgb, uint8_t *yuv, int32_t width, int32_t height, int32_t nframes,
+                        void *stream);
+
+/* The three HOST-buffer calls above with the picture side in format `f` (f == NULL or CM_PIX_RGB24: exactly the calls
+ * above).  For CM_PIX_YUV420P the picture buffers hold yuv420p frames: W wide on the input side, Wo wide on the output side;
+ * only those bytes cross the link, the conversions run on the device before the encoder and after the decoder. */
+int cm_encode_frames_host_fmt(cm_modem *m, const uint8_t *pic, uint8_t *comp, int64_t first_frame, int32_t nframes,
+                              const cm_pixfmt *f);
+int cm_decode_frames_host_fmt(cm_modem *m, const uint8_t *comp, uint8_t *pic, int64_t first_frame, int32_t nframes,
+                              const cm_pixfmt *f);
+int cm_transcode_frames_host_fmt(cm_modem *m, const uint8_t *pic_in, uint8_t *comp_out, uint8_t *pic_out,
+                                 int64_t first_frame, int32_t nframes, const cm_pixfmt *f);
+
 /* FilterFunction.__call__ (utils.py:28-36) on `nrows` independent rows of f->n samples each: causal IIR from zero
  * state, the input extended by f->shift copies of its last sample and the first f->shift outputs dropped.  `in` / `out`
  * are DEVICE buffers [nrows][f->n] of the given precision (float or double); f->rate is ignored.  Synchronises the
