@@ -15,6 +15,11 @@ static int launch_rows(cm_modem *m, IoArgs<T> io, cudaStream_t st, K kernel, F b
     if (rc) return rc;
     dim3 grid = cm_grid(io);
     int threads = cta_threads(m, warps_per_row * (R + extra_rows));
+    // cm_tune::min_warps may ask for more warps than the kernel is compiled for (k_niir_decode: 192 threads); the teams
+    // take whatever warps the CTA has, and a launch above the bound fails
+    cudaFuncAttributes fa;
+    CUDA_TRY(cudaFuncGetAttributes(&fa, kernel));
+    if (threads > fa.maxThreadsPerBlock) threads = fa.maxThreadsPerBlock & ~31;
     {
         LaunchTimer lt(m, timer_id, st);
         kernel<<<grid, threads, bytes(R), st>>>(params_of<T>(m), io);
