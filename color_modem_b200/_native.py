@@ -111,6 +111,7 @@ def load():
     lib.cm_decode_frames_host_fmt.argtypes = [vp, vp, vp, i64, i32, pf]
     lib.cm_transcode_frames_host_fmt.argtypes = [vp, vp, vp, vp, i64, i32, pf]
     lib.cm_measure_fma_peak.argtypes = [C.POINTER(C.c_double)]
+    lib.cm_pald_matrix.argtypes = [vp, vp, C.POINTER(C.c_int)]
     lib.cm_filter_rows.argtypes = [C.POINTER(Filter), C.c_int, vp, vp, i32, vp]
     lib.cm_launch_count.restype = C.c_int64
     lib.cm_timing_enable.argtypes = [vp, C.c_int]

@@ -1,5 +1,6 @@
 // C ABI of color_modem_b200 (include/color_modem_b200.h): handle management, filter-table construction and
 // dispatch to the per-family launchers (cm_qam.cu, cm_secam.cu, ...).  Host code only.
+#include <cuda_fp16.h>
 #include <math.h>
 #include <stdio.h>
 
@@ -379,6 +380,160 @@ static int upload(const std::vector<double> &src, void **dst) {
     return CM_OK;
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// PAL-D as a banded matrix product (cm_pald_mma.cu)
+// ------------------------------------------------------------------------------------------------------------
+// resample_poly of one line: out[j] = sum_i x[i] taps[half + j down - i up], zeros outside the line
+static void resample_line(const std::vector<double> &x, const cm_resampler &rs, std::vector<double> &out) {
+    const int n = (int)x.size(), nout = (n * rs.up + rs.down - 1) / rs.down;
+    out.assign(nout, 0.0);
+    for (int j = 0; j < nout; ++j) {
+        const int c = rs.half + j * rs.down;
+        const int lo = c - 2 * rs.half <= 0 ? 0 : (c - 2 * rs.half + rs.up - 1) / rs.up;
+        const int hi = c / rs.up < n - 1 ? c / rs.up : n - 1;
+        double acc = 0.0;
+        for (int i = lo; i <= hi; ++i) acc += x[i] * rs.taps[c - i * rs.up];
+        out[j] = acc;
+    }
+}
+
+// one IIR use-site on one line: `shift` copies of the last sample appended, second-order sections (DF-II-T, zero state),
+// the first `shift` outputs dropped (oracle/dsp.py: Filt)
+static void iir_line(std::vector<double> &x, const cm_filter &f) {
+    const size_t n = x.size();
+    std::vector<double> y(x);
+    y.resize(n + f.shift, x[n - 1]);
+    for (int s = 0; s < f.nsec; ++s) {
+        const double *c = f.sos[s];
+        double z1 = 0.0, z2 = 0.0;
+        for (double &v : y) {
+            const double in = v, out = c[0] * in + z1;
+            z1 = c[1] * in - c[3] * out + z2;
+            z2 = c[2] * in - c[4] * out;
+            v = out;
+        }
+    }
+    for (size_t i = 0; i < n; ++i) x[i] = y[i + f.shift];
+}
+
+static bool pald_kind(const cm_desc &d) {
+    return d.kind == CM_KIND_PAL_D || (d.kind == CM_KIND_PAL_3D && !(d.flags & (CM_FLAG_PAL3D_SIN | CM_FLAG_PAL3D_COS)));
+}
+
+// The linear map of pass 1 of the PAL-D decoder (k_qam_rows2<PALD> before the row's phase rotation), from the signal of
+// the W composite samples to the planes of each sample x: M[i * 4W + 4x + plane], planes a', b', LPpre a', LPpre b'.
+// Restated on unit impulses: up2, band-pass, down2, up2, the table carrier (sin for a', cos for b'), the AM low-pass,
+// down2, then the encoder's chroma low-pass.
+static void pald_matrix(const cm_desc &d, std::vector<double> &M) {
+    const int W = d.width;
+    const cm_resampler &up = d.resamplers[QR_UP2], &dn = d.resamplers[QR_DOWN2];
+    const cm_filter &fbp = d.filters[QF_BP2X], &flp = d.filters[QF_PALD_LP], &fpre = d.filters[QF_PRE_LP];
+    std::vector<double> car[2];
+    car[0].resize(2 * W);
+    car[1].resize(2 * W);
+    for (int j = 0; j < 2 * W; ++j) {      // as build_carrier_table
+        const unsigned long long ph = (unsigned long long)j * d.phases[QP_STEP2X];
+        const double turns = (double)(long long)ph * 5.421010862427522170e-20;
+        car[0][j] = sin(6.283185307179586476925 * turns);
+        car[1][j] = cos(6.283185307179586476925 * turns);
+    }
+    M.assign((size_t)W * 4 * W, 0.0);
+    std::vector<double> x(W), g, c, g2, pr(2 * W), a;
+    for (int i = 0; i < W; ++i) {
+        std::fill(x.begin(), x.end(), 0.0);
+        x[i] = 1.0;
+        resample_line(x, up, g);
+        iir_line(g, fbp);
+        resample_line(g, dn, c);
+        resample_line(c, up, g2);
+        for (int t = 0; t < 2; ++t) {
+            for (int j = 0; j < 2 * W; ++j) pr[j] = g2[j] * car[t][j];
+            iir_line(pr, flp);
+            resample_line(pr, dn, a);
+            double *row = &M[(size_t)i * 4 * W];
+            for (int s = 0; s < W; ++s) row[4 * s + t] = a[s];
+            iir_line(a, fpre);
+            for (int s = 0; s < W; ++s) row[4 * s + 2 + t] = a[s];
+        }
+    }
+}
+
+// Reach of M (pald_matrix) around the diagonal: output sample x depends on the inputs [x - lo, x + hi], to 2^-26 of the
+// largest coefficient of its plane.
+static void pald_band(const std::vector<double> &M, int W, int &lo, int &hi) {
+    double mx[4] = {0, 0, 0, 0};
+    for (size_t k = 0; k < M.size(); ++k) mx[k & 3] = fmax(mx[k & 3], fabs(M[k]));
+    lo = hi = 0;
+    for (int i = 0; i < W; ++i)
+        for (int n = 0; n < 4 * W; ++n)
+            if (fabs(M[(size_t)i * 4 * W + n]) > ldexp(mx[n & 3], -26)) {
+                const int x = n >> 2;
+                if (x - i > lo) lo = x - i;
+                if (i - x > hi) hi = i - x;
+            }
+}
+
+// B operand of k_pald_mma (cm_host.h: PaldMmaArgs) for a float32 PAL-D handle whose band fits the compiled window; leaves
+// the handle without it (the two-pass kernels serve it) otherwise.  The level map is folded in: the composite signal is
+// (5 u / 255 - 1) / 3 for the byte u, so the planes are u . (5 / 765) M - (1 / 3) colsum(M).  Each column is scaled by a
+// power of two (largest coefficient near 1000) and split into FP16 hi + lo.
+static int plan_pald_mma(cm_modem *m) {
+    const cm_desc &d = m->desc;
+    const int W = d.width;
+    if (m->precision != CM_FP32 || !m->tune.pald_mma || m->tune.onepass || m->tune.rows_v1 || !pald_kind(d) ||
+        !m->pf.row_geo || d.comp_width != W || d.out_width != W || d.resamplers[QR_UP2].ntaps <= 0 ||
+        d.resamplers[QR_DOWN2].ntaps <= 0)
+        return CM_OK;
+    std::vector<double> M;
+    pald_matrix(d, M);
+    int lo = 0, hi = 0;
+    pald_band(M, W, lo, hi);
+    if (lo > CM_PALD_KPRE || hi > CM_PALD_KW - CM_PALD_KPRE - CM_PALD_TS) return CM_OK;
+    const int ntiles = (W + CM_PALD_TS - 1) / CM_PALD_TS, kc = CM_PALD_KW / 8, N = CM_PALD_N;
+    std::vector<uint16_t> B((size_t)ntiles * 2 * CM_PALD_KW * N, 0);
+    std::vector<float> cs((size_t)ntiles * 2 * N, 0.0f);
+    for (int tile = 0; tile < ntiles; ++tile) {
+        const int xs = tile * CM_PALD_TS - CM_PALD_KPRE;
+        for (int n = 0; n < N; ++n) {
+            const int x = tile * CM_PALD_TS + (n >> 2), col = 4 * x + (n & 3);
+            float *inv = &cs[(size_t)tile * 2 * N + n], *bias = inv + N;
+            *inv = 1.0f;
+            if (x >= W) continue;
+            double mx = 0.0, sum = 0.0;
+            for (int i = 0; i < W; ++i) sum += M[(size_t)i * 4 * W + col];
+            for (int k = 0; k < CM_PALD_KW; ++k)
+                if (xs + k >= 0 && xs + k < W) mx = fmax(mx, fabs(M[(size_t)(xs + k) * 4 * W + col]) * (5.0 / 765.0));
+            const double scale = mx > 0.0 ? ldexp(1.0, (int)floor(log2(1000.0 / mx))) : 1.0;
+            *inv = (float)(1.0 / scale);
+            *bias = (float)(-sum / 3.0);
+            for (int k = 0; k < CM_PALD_KW; ++k) {
+                if (xs + k < 0 || xs + k >= W) continue;
+                const double r = M[(size_t)(xs + k) * 4 * W + col] * (5.0 / 765.0) * scale;
+                const __half h = __float2half_rn((float)r);
+                const __half l = __float2half_rn((float)(r - (double)__half2float(h)));
+                const size_t at = ((size_t)(tile * 2) * kc + k / 8) * N * 8 + (size_t)n * 8 + (k & 7);
+                B[at] = __half_as_ushort(h);
+                B[at + (size_t)kc * N * 8] = __half_as_ushort(l);
+            }
+        }
+    }
+    CUDA_TRY(cudaMalloc(&m->d_mma_b, B.size() * sizeof(uint16_t)));
+    CUDA_TRY(cudaMemcpy(m->d_mma_b, B.data(), B.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMalloc(&m->d_mma_cs, cs.size() * sizeof(float)));
+    CUDA_TRY(cudaMemcpy(m->d_mma_cs, cs.data(), cs.size() * sizeof(float), cudaMemcpyHostToDevice));
+    return CM_OK;
+}
+
+// Test hook: the matrix of pald_matrix (W x 4W, float64, row-major) and its band (lo, hi) for a PAL-D handle.
+extern "C" int cm_pald_matrix(const cm_modem *m, double *out, int *band) {
+    if (!m || !pald_kind(m->desc)) return fail(CM_ERR_UNSUPPORTED, "not a PAL-D handle%s");
+    std::vector<double> M;
+    pald_matrix(m->desc, M);
+    if (out) memcpy(out, M.data(), M.size() * sizeof(double));
+    if (band) pald_band(M, m->desc.width, band[0], band[1]);
+    return CM_OK;
+}
+
 extern "C" int cm_abi_version(void) { return CM_ABI_VERSION; }
 extern "C" int cm_sizeof_desc(void) { return (int)sizeof(cm_desc); }
 extern "C" const char *cm_last_error(void) { return g_err; }
@@ -448,6 +603,7 @@ extern "C" int cm_create(const cm_desc *desc, int precision, cm_modem **out) {
         if (m->tune.mac_threads < 32) m->tune.mac_threads = 32;
         if (m->tune.mac_threads > CM_NTHREADS) m->tune.mac_threads = CM_NTHREADS;       // the kernels' launch bound
         if (const char *e = getenv("CM_OVERLAP")) m->tune.overlap = atoi(e);
+        if (const char *e = getenv("CM_PALD_MMA")) m->tune.pald_mma = atoi(e) != 0;
     }
     cudaError_t e = cudaGetDevice(&m->device);
     if (e != cudaSuccess) { delete m; return fail(CM_ERR_CUDA, "cudaGetDevice: %s", cudaGetErrorString(e)); }
@@ -564,6 +720,7 @@ extern "C" int cm_create(const cm_desc *desc, int precision, cm_modem **out) {
         m->pf.ctab = (const float *)m->d_ctab;
         m->pf.row_geo = row_geo ? row_geo : (sec_geo ? sec_geo : niir_geo);
         m->pf.enc_geo = enc_geo;
+        if (rc == CM_OK) rc = plan_pald_mma(m);
     } else {
         rc = upload<double>(tab, &m->d_tab);
         if (rc == CM_OK) rc = upload<double>(taps, &m->d_taps);
@@ -590,6 +747,8 @@ extern "C" void cm_destroy(cm_modem *m) {
     cudaFree(m->d_taps);
     cudaFree(m->d_ctab);
     cudaFree(m->d_ptab);
+    cudaFree(m->d_mma_b);
+    cudaFree(m->d_mma_cs);
     if (m->last_use) cudaEventDestroy(m->last_use);
     if (m->s2) cudaStreamDestroy(m->s2);
     for (int i = 0; i < 2; ++i) {

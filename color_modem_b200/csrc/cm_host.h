@@ -19,7 +19,7 @@ void cm_count_launch();
     } while (0)
 
 // Tuning knobs of a handle.  Read ONCE, in cm_create, from the environment (CM_ONEPASS, CM_ROWS_V1, CM_RPC, CM_CHUNK,
-// CM_HOST_CHUNK, CM_ROWS_MAX, CM_MIN_WARPS, CM_OVERLAP: A/B aids of tools/ab.py and of the alternative-path parity tests) — no launch
+// CM_HOST_CHUNK, CM_ROWS_MAX, CM_MIN_WARPS, CM_OVERLAP, CM_PALD_MMA: A/B aids of tools/ab.py and of the alternative-path parity tests) — no launch
 // path calls getenv.
 struct cm_tune {
     bool onepass = false;      // legacy multi-row halo kernels instead of the two-pass row kernels
@@ -33,7 +33,24 @@ struct cm_tune {
     int rows_max = 0;          // upper bound of rows per CTA of the multi-row kernels (0: none)
     int min_warps = 2;         // fewest warps per CTA of the multi-row kernels
     int mac_threads = 128;     // threads per CTA of the MAC kernels (CM_MAC_THREADS)
+    bool pald_mma = true;      // PAL-D on the tensor cores where it serves the call (CM_PALD_MMA=0: the two-pass kernels)
     int overlap = 0;           // pass 2 of chunk i on a second stream under pass 1 of chunk i + 1 (measured: no gain, DESIGN.md section 5)
+};
+
+// PAL-D on the tensor cores (cm_pald_mma.cu): column tiles of TS output samples, N = 4 TS plane columns (a', b', LPpre a',
+// LPpre b' of each sample), a K window of KW composite samples starting KPRE before the tile
+#define CM_PALD_TS 32
+#define CM_PALD_N (4 * CM_PALD_TS)
+#define CM_PALD_KW 160
+#define CM_PALD_KPRE 96
+
+struct PaldMmaArgs {
+    const uint16_t *b;      // [tile][hi | lo][KW / 8][N][8] FP16, the UMMA K-major layout without swizzle
+    const float *cs;        // [tile][inverse column scale | bias][N]
+    long long total;        // rows in the list of the call
+    int per_frame;          // list rows per frame: len_a of the field of out_begin, then the other field's
+    int len_a, row_a;       // rows listed for the field of out_begin, the first of them (the predecessor out_begin - 2)
+    int nblocks;            // row tiles of 127 output lanes
 };
 
 struct cm_modem {
@@ -51,6 +68,8 @@ struct cm_modem {
     void *d_taps = nullptr;
     void *d_ctab = nullptr;
     void *d_ptab = nullptr;
+    void *d_mma_b = nullptr;    // PAL-D tensor-core kernel: B tiles and column scale / bias (plan_pald_mma); nullptr: not served
+    void *d_mma_cs = nullptr;
     bool timing = false;
     unsigned long long *phase_prof = nullptr;
     // pairing scratch of the line-sequential decoders (grown on demand); one per host-path stream (+ slot 0 for
@@ -190,3 +209,4 @@ template <typename T> int proto_encode(cm_modem *m, IoArgs<T> io, cudaStream_t s
 template <typename T> int proto_decode(cm_modem *m, IoArgs<T> io, cudaStream_t st);
 template <typename T> int mac_encode(cm_modem *m, IoArgs<T> io, cudaStream_t st);
 template <typename T> int mac_decode(cm_modem *m, IoArgs<T> io, cudaStream_t st);
+int launch_pald_mma(cm_modem *m, IoArgs<float> io, cudaStream_t st);

@@ -173,6 +173,11 @@ template <typename T, int MODE>
 int launch_rows_pair(cm_modem *m, IoArgs<T> io, cudaStream_t st) {
     const DevParams<T> &p = params_of<T>(m);
     if (io.out_count <= 0) return CM_OK;
+    if constexpr (MODE == PAIR_PALD && IsF32<T>::value) {
+        // u8 composite (exact in FP16) without the (y, u, v) diversion of the non-default knobs: one kernel on the
+        // tensor cores when the handle has its band matrix (cm_api.cu: plan_pald_mma)
+        if (m->d_mma_b && io.in_u8 && !io.yuv) return launch_pald_mma(m, io, st);
+    }
     size_t b1 = (128 + (size_t)p.n1p + 6 * (size_t)p.hb2) * sizeof(T);
     const bool teams = needs_teams(p);
     constexpr bool kPald = MODE == PAIR_PALD;
