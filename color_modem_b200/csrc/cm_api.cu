@@ -882,6 +882,10 @@ static int run_ex(cm_modem *m, bool encode, const cm_window *win, const uint8_t 
     if (nframes == 0) return CM_OK;                    // an empty batch may come with null buffers
     if ((in_u8 == nullptr) == (in_f == nullptr)) return fail(CM_ERR_INVALID, "exactly one input buffer required%s");
     if (!out_u8 && !out_f) return fail(CM_ERR_INVALID, "no output buffer%s");
+    // u8 frames move in 32-bit words, float frames in vectors of four samples (cm_fir.cuh: ld4 / st4; float4 for float)
+    const uintptr_t falign = sizeof(T) == 4 ? 16 : alignof(T);
+    if ((((uintptr_t)in_u8 | (uintptr_t)out_u8) & 3) || (((uintptr_t)in_f | (uintptr_t)out_f) & (falign - 1)))
+        return fail(CM_ERR_INVALID, "misaligned frame buffer%s");
     IoArgs<T> io;
     memset(&io, 0, sizeof(io));
     io.in_u8 = in_u8;

@@ -131,6 +131,7 @@ class GpuModem(object):
                     or not t.is_contiguous()):
                 raise ValueError('output must be a contiguous CUDA %s tensor of shape [%d, %s] on %s' % (
                     dtype, n, ', '.join(map(str, tail)), src.device))
+            self._check_aligned(t)
 
     def encode_frames(self, rgb, first_frame=0, out=None, out_float=None):
         """rgb: CUDA uint8 tensor [N, H, W, 3] -> composite uint8 [N, H, Wc] (ImageModem.modulate, image.py:27-56)."""
@@ -166,6 +167,17 @@ class GpuModem(object):
     def _check(t, dtype, tail):
         if not t.is_cuda or t.dtype != dtype or tuple(t.shape[1:]) != tuple(tail) or not t.is_contiguous():
             raise ValueError('expected a contiguous CUDA %s tensor of shape [N, %s]' % (dtype, ', '.join(map(str, tail))))
+        GpuModem._check_aligned(t)
+
+    @staticmethod
+    def _check_aligned(t):
+        """The kernels move u8 frames in 32-bit words and float frames in vectors of four samples (16 bytes for float32,
+        8-byte words for float64): a contiguous view at another storage offset is refused (include/color_modem_b200.h)."""
+        torch = _torch()
+        align = 4 if t.dtype == torch.uint8 else (16 if t.dtype == torch.float32 else 8)
+        if t.numel() and t.data_ptr() % align:
+            raise ValueError('frame buffer at %#x is not %d-byte aligned (a view at storage offset %d)' % (
+                t.data_ptr(), align, t.storage_offset()))
 
     # ---- frame batches with host buffers (H2D + kernels + D2H inside the native call) ------------------------
     @staticmethod

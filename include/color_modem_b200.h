@@ -160,9 +160,11 @@ int cm_sizeof_desc(void);
 const char *cm_last_error(void);
 int cm_device_info(int *sm_count, int *cc_major, int *cc_minor);
 
-/* Line widths (width, comp_width, out_width) must be multiples of 4 samples and frame pointers 4-byte aligned: the kernels
- * move four samples per 32-bit / 96-bit / 128-bit access.  (The reference accepts any width: image.py:27-84.)  The tuning
- * knobs of a handle are read from the environment here, once. */
+/* Line widths (width, comp_width, out_width) must be multiples of 4 samples, u8 frame pointers 4-byte aligned and float
+ * frame pointers 16-byte (float) / 8-byte (double) aligned: the kernels move four samples per 32-bit / 96-bit / 128-bit
+ * access (a float vector of four samples in one access).  cm_encode_ex / cm_decode_ex refuse a misaligned frame pointer
+ * with CM_ERR_INVALID before any launch.  (The reference accepts any width: image.py:27-84.)  The tuning knobs of a handle
+ * are read from the environment here, once. */
 int cm_create(const cm_desc *desc, int precision, cm_modem **out);
 void cm_destroy(cm_modem *m);
 

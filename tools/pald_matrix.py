@@ -7,7 +7,7 @@ matrix, checks linearity, and evaluates the two-term FP16 split that k_pald_mma 
 multiplies with on random u8 rows.  With --library it also compares the library's own matrix (cm_pald_matrix, built on
 the host from the handle's filters; needs the built library and a GPU for the handle).
 
-    python tools/pald_matrix.py [--width 720] [--library]
+    python tools/pald_matrix.py [--variant PAL] [--standard GERBER_625] [--width 720] [--library]
 """
 import argparse
 import os
@@ -21,9 +21,9 @@ import oracle  # noqa: E402
 KPRE, KW, TS = 96, 160, 32        # the compiled window of k_pald_mma (cm_host.h: CM_PALD_*)
 
 
-def oracle_matrix(w, h=576):
+def oracle_matrix(w, h=576, variant='PAL', standard='GERBER_625'):
     """M[i, 4 x + plane]: plane (a', b', LPpre a', LPpre b') of sample x for a unit impulse at input i."""
-    m = oracle.build(oracle.ModemSpec('pal_d', 'PAL', w, h))
+    m = oracle.build(oracle.ModemSpec('pal_d', variant, w, h, standard))
     ex = m.qam.extract(np.eye(w))
     a, b = m._am(ex, 0.0), m._am(ex, 0.5 * np.pi)
     planes = np.stack([a, b, m.qam.pre_lp(a), m.qam.pre_lp(b)], axis=-1)    # [i, x, plane]
@@ -57,12 +57,12 @@ def fp16_split_error(M, rows=256, seed=1):
     return float(np.abs(got - exact).max()), float(np.abs(exact).max())
 
 
-def library_matrix(w, h=576):
+def library_matrix(w, h=576, variant='PAL', standard='GERBER_625'):
     import ctypes as C
     from color_modem_b200 import _native as N
     from color_modem_b200.color import pal
     from color_modem_b200.line import LineConfig, LineStandard as LS
-    modem = pal.PalDModem(LineConfig((w, h), LS.GERBER_625))
+    modem = pal.PalDModem(LineConfig((w, h), getattr(LS, standard)), getattr(pal.PalVariant, variant))
     M = np.zeros((w, 4 * w))
     bd = (C.c_int * 2)()
     N.check(N.load().cm_pald_matrix(modem._handle(), M.ctypes.data, bd))
@@ -71,18 +71,20 @@ def library_matrix(w, h=576):
 
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
+    ap.add_argument('--variant', default='PAL', choices=('PAL', 'PAL_M', 'PAL_N'))
+    ap.add_argument('--standard', default='GERBER_625', help='line standard (PAL_M: NTSC_525)')
     ap.add_argument('--width', type=int, default=720)
     ap.add_argument('--library', action='store_true', help='compare with the library matrix (needs a GPU)')
     a = ap.parse_args()
-    M, m = oracle_matrix(a.width)
+    M, m = oracle_matrix(a.width, variant=a.variant, standard=a.standard)
     x = np.random.default_rng(0).uniform(0, 1, a.width)
     lin = np.abs(x @ M[:, 0::4] - m._am(m.qam.extract(x[None]), 0.0)[0]).max()
     lo, hi = band(M)
     err, top = fp16_split_error(M)
-    print('width %d: linearity %.1e, band [x - %d, x + %d] at 2^-26 (window [x - %d, x + %d]), fp16 x2 error %.2e '
-          '(planes up to %.2f)' % (a.width, lin, lo, hi, KPRE, KW - KPRE - TS, err, top))
+    print('%s (%s) width %d: linearity %.1e, band [x - %d, x + %d] at 2^-26 (window [x - %d, x + %d]), fp16 x2 error %.2e '
+          '(planes up to %.2f)' % (a.variant, a.standard, a.width, lin, lo, hi, KPRE, KW - KPRE - TS, err, top))
     if a.library:
-        L, bd = library_matrix(a.width)
+        L, bd = library_matrix(a.width, variant=a.variant, standard=a.standard)
         print('library: band [x - %d, x + %d], largest difference from the oracle %.2e' % (bd[0], bd[1],
                                                                                           np.abs(L - M).max()))
 
